@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps K --warmup W                  # this repo's CUDA path
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...   # one rank per GPU
     python bench.py --impl reference --gpus N --steps K --warmup W  # CPU arm (oracle port, host cores)
+    python bench.py ... --dump-outputs DIR                          # also the last timed step's outputs, DIR/<name>.npy
 
 A "step" is one pass of the hot path over the whole synthetic workload (--config: BASELINE config 2 by default:
 30x ONT whole genome, 24 GRCh38-length contigs, ~6M reads at --scale 1; 1 = one 1 Mb contig, 3 = 60x HiFi --mosaic,
@@ -194,17 +195,8 @@ def cpu_sample(blk, cfg, ccfg, threads, target_bp=6e9):
 
 
 def python_reference_baseline():
-    """The reference's own Python code timed in this run when its tree is present (build container, or $SNIFFLES_REFERENCE_SRC on the box);
-    otherwise the committed measurement of the build container, labelled as such (BASELINE.md §3).  Never a silent quote."""
-    try:
-        sys.path.insert(0, os.path.join(ROOT, "oracle", "pyref"))
-        import timing
-        if timing.available():
-            m = timing.measure()
-            m["where"] = "this run"
-            return m
-    except Exception as e:
-        log(f"[bench] python reference leg failed: {e}")
+    """The committed measurement of the reference's own Python code (oracle/pyref/timing.py, BASELINE.md §3), labelled as measured
+    elsewhere: the benchmark reads nothing outside this repository.  Never a silent quote."""
     p = os.path.join(ROOT, "tests", "expected", "python_reference_timing.json")
     if os.path.exists(p):
         with open(p) as f:
@@ -243,6 +235,59 @@ def committed_hashes():
         with open(p) as f:
             return json.load(f)
     return {}
+
+
+DUMP_BYTES = 60_000_000         # --dump-outputs: array bytes in all, under 64 MB with the .npy headers
+DUMP_SEED = 1729
+
+
+def _float_columns(a, name):
+    """{file name: column} of a plain or structured array, rows first: float32 where that is exact (integers of up to 16 bits,
+    float32), float64 otherwise; a 64-bit integer column (hashes, arena offsets) becomes two exact columns `<name>_hi`, `<name>_lo`.
+    Every value written is finite: a floating-point column (where NaN stands for an undefined result, e.g. the stdev of one value)
+    has its non-finite values written as 0 and a column `<name>_nonfinite` saying which they were: 0 finite, 1 NaN, 2 +inf, 3 -inf."""
+    if a.dtype.names:
+        out = {}
+        for f in a.dtype.names:
+            if not f.startswith("_"):
+                out.update(_float_columns(a[f], f"{name}.{f}"))
+        return out
+    if a.dtype.kind in "iu" and a.dtype.itemsize == 8:
+        u = a.astype("<u8")
+        return {f"{name}_hi": (u >> np.uint64(32)).astype(np.float64), f"{name}_lo": (u & np.uint64(0xFFFFFFFF)).astype(np.float64)}
+    out = a.astype(np.float32 if a.dtype.itemsize <= 2 or a.dtype == np.float32 else np.float64)
+    if a.dtype.kind != "f":
+        return {name: out}
+    kind = np.select([np.isnan(out), out == np.inf, out == -np.inf], [1, 2, 3], 0).astype(np.float32)
+    return {name: np.where(kind == 0, out, 0).astype(out.dtype), f"{name}_nonfinite": kind}
+
+
+def dump_outputs(dirname, tables, prefix=""):
+    """--dump-outputs: every array of `tables` ({name: array, rows first}) as DIR/<prefix><name>[.<field>].npy.  A table larger than its
+    share of DUMP_BYTES (the smaller tables are kept whole first) keeps a seeded sample of its rows, the same rows for the same row
+    count, whose indices go to <name>.rows.npy.  The dump lets two builds be compared output for output on identical inputs."""
+    os.makedirs(dirname, exist_ok=True)
+    tables = {k: np.asarray(a) for k, a in tables.items() if a is not None}
+    row_bytes = {k: sum(c.itemsize * max(1, c[:1].size) for c in _float_columns(a[:1], k).values()) for k, a in tables.items()}
+    left, order = DUMP_BYTES, sorted(tables, key=lambda k: len(tables[k]) * row_bytes[k])
+    for i, k in enumerate(order):
+        a, share = tables[k], left // (len(order) - i)
+        if len(a) * row_bytes[k] > share:
+            m = share // (row_bytes[k] + 8)
+            rows = np.sort(np.random.default_rng(DUMP_SEED).choice(len(a), m, replace=False))
+            log(f"[bench] --dump-outputs: {k} sampled, {m} of {len(a)} rows")
+            np.save(os.path.join(dirname, f"{prefix}{k}.rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+            left -= 8 * m
+        for name, col in _float_columns(a, k).items():
+            np.save(os.path.join(dirname, f"{prefix}{name}.npy"), col)
+            left -= col.nbytes
+
+
+def result_tables(res):
+    """the arrays a caller of Context.run / oracle.run receives"""
+    return {"leads": res.leads, "cand": res.cand, "cand_leads": res.cand_leads, "rnames": res.rnames, "rn_off": res.rn_off,
+            "task_cov_mean": res.task_cov_mean, "alt": res.alt}
 
 
 PARITY_FIELDS = ["task", "svtype", "pos", "end", "svlen", "support", "qual", "precise", "fwd", "rev", "cov_upstream", "cov_start", "cov_center", "cov_end",
@@ -289,8 +334,8 @@ def run_reference(args):
         info, abp, dt = cpu_sample(blk, cfg, ccfg, ncores, target_bp=args.cpu_sample_gbp * 1e9)
         if i >= args.warmup:
             per_step.append(dt)
-        if i == 0 and dt * (args.warmup + args.steps) > 240:     # keep the whole run within minutes
-            args.steps = max(1, min(args.steps, int(240 / dt) - args.warmup))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, result_tables(cpu_sample.last_result))
     ms = 1e3 * sum(per_step) / len(per_step)
     val = abp / (ms / 1e3) / 1e9
     info["value"] = val
@@ -403,6 +448,8 @@ def run_b200(args):
     clocks = sampler.stop()
     launches = ctx.launch_count() - launches0
     reruns = ctx.rerun_count() - reruns0
+    if args.dump_outputs:           # before the runs below reuse the library's output buffers that `res` views
+        dump_outputs(args.dump_outputs, result_tables(res), f"rank{rank}." if world > 1 else "")
     # max over ranks
     tt = torch.tensor([dev_ms, wall * 1e3, float(abp_local)], device="cuda", dtype=torch.float64)
     if dist is not None:
@@ -600,6 +647,8 @@ def run_combine(args):
     torch.cuda.synchronize()
     wall = time.perf_counter() - t1
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("cand_group", "emit_chunk", "emit_ord", "cov_non"), out)))
     ms_per_step = wall / args.steps * 1e3
     n_groups = int((out[1][:n] >= 0).sum())
     h2d = sum(int(arrays[k].nbytes) for k in ("chains", "chunks", "pos", "svlen", "sample", "mate_contig", "mate_pos", "block_start", "cov", "alt", "alt_off", "alt_len"))
@@ -715,6 +764,8 @@ def run_ingest(args):
         for nm, ms, _b in ctx.timings():
             stage[nm] = stage.get(nm, 0.0) + ms / args.steps
     clocks = sampler.stop()
+    if args.dump_outputs:           # the record block the last load built in device memory
+        dump_outputs(args.dump_outputs, dict(zip(("rec", "cigar16", "var", "seq"), ctx.ingest_fetch())))
     kern_ms = sum(stage.get(k, 0.0) for k in ("inflate", "walk_records", "parse_records", "record_sizes", "pack_records"))
     e2e_ms = wall / args.steps * 1e3
     # the whole path fed compressed bytes: ingest + stages A-C, candidates back on the host
@@ -757,7 +808,11 @@ def main():
     ap.add_argument("--e2e-full-seq", action="store_true", help="e2e: copy the whole seq arena every step instead of the on-demand slices")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--write-hash", action="store_true", help="1 GPU: when the call set equals the oracle's, write its hash to gpurun_out/callset_hashes.json (to be committed under tests/expected/)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the arrays the timed path returned in its last step as DIR/<name>.npy "
+                    "(float32 / float64, at most 64 MB: larger outputs are sampled with a fixed seed), to compare two builds on identical inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "b200":
         log("[bench] note: timing rules ask for >= 3 warm-up steps")
     import __graft_entry__ as g

@@ -1,7 +1,7 @@
 """Times the UNMODIFIED reference (build_leadtab + call_candidates + finalize_candidates, parallel.py:90-201) on seeded
-synthetic blocks, htslib decode excluded (the reads are materialised before the clock starts) — the `cpu_baseline_python`
-leg of bench.py (BASELINE.md §3).  TEST / BASELINE INFRASTRUCTURE: runs only where the reference tree exists
-(/root/reference/src or $SNIFFLES_REFERENCE_SRC); bench.py falls back to the committed measurement otherwise.
+synthetic blocks, htslib decode excluded (the reads are materialised before the clock starts) — the committed measurement
+bench.py reports as `cpu_baseline_python` (BASELINE.md §3).  TEST / BASELINE INFRASTRUCTURE: runs only where the reference
+tree exists (harness.REFERENCE_SRC).
 
     python oracle/pyref/timing.py --write          # refresh tests/expected/python_reference_timing.json (build container)
 """
